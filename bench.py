@@ -2,7 +2,11 @@
 """Benchmark of the pseudo-label hot path (BASELINE.json: "k-reciprocal Jaccard+DBSCAN sec at N=32,621").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload rerank|cm|pass|market|scale100k|scale250k|hard]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR writes what the last timed step computed as DIR/<name>.npy (see dump_outputs); the inputs are seeded,
+so two builds run with the same arguments can be compared output for output.
 
 A step = one full pass: kNN (tcgen05 GEMM + fused top-K + exact re-score) -> k-reciprocal sets ->
 expansion -> Gaussian weights -> k2 query expansion -> inverted index -> sparse Jaccard eps-graph ->
@@ -150,6 +154,46 @@ def rank_sha256(rank):
     import hashlib
     import numpy as np
     return hashlib.sha256(np.ascontiguousarray(np.asarray(rank).astype(np.int32)).tobytes()).hexdigest()
+
+
+DUMP_BYTES = 64 << 20                  # --dump-outputs writes at most this much in all,
+DUMP_ARRAY_BYTES = DUMP_BYTES // 8     # and at most this much per output (a step has at most six outputs)
+
+
+def host_outputs(arrays):
+    """Host copies of one step's outputs (None entries dropped), taken before later passes reuse their buffers."""
+    return {name: a.detach().cpu().numpy() for name, a in arrays.items() if a is not None}
+
+
+def dump_outputs(out_dir, arrays):
+    """Write every output as out_dir/<name>.npy: float64 stays float64, other floats become float32, integers and flags
+    float64 (exact below 2^53).  An output larger than DUMP_ARRAY_BYTES keeps a fixed, seeded sample of its rows, whose
+    indices go to out_dir/<name>_rows.npy: the same rows for the same shape, whichever build wrote them."""
+    import numpy as np
+    files = {}
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        a = a.astype(np.float32 if a.dtype in (np.float16, np.float32) else np.float64).reshape(a.shape or (1,))
+        if a.nbytes > DUMP_ARRAY_BYTES:
+            m = DUMP_ARRAY_BYTES // (a.nbytes // a.shape[0] + 8)
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], m, replace=False))
+            files[name + "_rows"] = rows.astype(np.float64)
+            a = a[rows]
+        files[name] = a
+    total = sum(a.nbytes for a in files.values())
+    if total > DUMP_BYTES:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in files.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def pass_outputs(out):
+    """What a caller of pipeline / sharded.pseudo_labels receives: labels, core-point flags, the number of clusters, the
+    centroids when the workload asks for them, and the neighbour lists with their search keys (the rank's own rows)."""
+    st = out["state"]
+    return {"labels": out["labels"], "core": out["core"], "num_clusters": out["num_clusters"],
+            "centroids": out.get("centroids"), "neighbors": st.rank, "neighbor_keys": st.rank_key}
 
 
 def host_mem_gb():
@@ -454,17 +498,19 @@ def run_cm(args):
     hbat = [(a.pin_memory(), b.pin_memory()) for a, b in batches]
 
     def step(inp, tgt):
+        """One step; returns the mean loss, the per-sample losses and the inputs, whose .grad the backward filled."""
         inp = inp.requires_grad_(True)
-        loss = mem(inp, tgt).mean()
-        loss.backward()
-        return loss
+        loss = mem(inp, tgt)
+        mean = loss.mean()
+        mean.backward()
+        return mean, loss, inp
 
     sampler = ClockSampler(dev.index or 0)
     sampler.start()
     for i in range(max(args.warmup, 3)):
         step(*dbat[i % 8])
     torch.cuda.synchronize()
-    steps = max(args.steps, 200)                     # a step lasts tens of microseconds: time enough of them
+    steps = args.steps                               # a step lasts tens of microseconds: --steps in the hundreds times enough
     l0 = _lib.launch_count()
     _lib.profiler.start()
     for i in range(8):
@@ -476,16 +522,20 @@ def run_cm(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(steps):
-        step(dbat[i % 8][0].detach(), dbat[i % 8][1])
+        _, loss, inp = step(dbat[i % 8][0].detach(), dbat[i % 8][1])
     e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / steps
+    if args.dump_outputs:                            # before the end-to-end steps move the centroids on
+        dumped = host_outputs({"loss": loss, "input_grad": inp.grad, "features": mem.features})
     t0 = time.perf_counter()
     for i in range(steps):
         a, b = hbat[i % 8]
-        lv = float(step(a.to(dev, non_blocking=True), b.to(dev, non_blocking=True)).item())
+        lv = float(step(a.to(dev, non_blocking=True), b.to(dev, non_blocking=True))[0].item())
     e2e_s = (time.perf_counter() - t0) / steps
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dumped)
     peaks = measured_peaks()
     nbytes = 4.0 * (2 * B * D + 2 * C * D + B * C)
     kernel_ms = {k: round(v[1] / 8, 5) for k, v in sorted(prof.items(), key=lambda kv: -kv[1][1])}
@@ -545,7 +595,14 @@ def main():
     ap.add_argument("--workload", default="rerank", choices=["cm"] + list(WORKLOADS),
                     help="rerank = BASELINE configs[1] (the headline); cm = configs[2]; pass = configs[3]; "
                          "market = configs[0]; scale100k / scale250k = configs[4]; hard = the parity set")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of the last one as DIR/<name>.npy (float32 / float64, "
+                         "at most 64 MB in all; larger outputs as a fixed, seeded sample of rows)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path; it does not apply to --impl reference")
     args.warmup = max(args.warmup, 0)
     pin_host_threads()
     if args.workload == "cm":
@@ -625,6 +682,8 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:                     # `out` is still the last timed pass
+        dump_outputs(args.dump_outputs, host_outputs(pass_outputs(out)))
     # ---- per-entry-point CUDA-event times (separate passes: the event pairs cost a few microseconds per launch) ----
     p_steps = max(3, min(args.steps, 10))
     l0 = _lib.launch_count()

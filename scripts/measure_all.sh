@@ -4,7 +4,7 @@
 tag=${1:-r02_v3}
 out=gpurun_out
 mkdir -p $out
-python bench.py --workload cm > $out/bench_r02_cm.json 2> $out/cm.err
+python bench.py --workload cm --steps 200 > $out/bench_r02_cm.json 2> $out/cm.err
 python bench.py --workload pass --steps 30 --warmup 5 > $out/bench_r02_pass_n1.json 2> $out/pass.err
 python bench.py --workload market --steps 30 --warmup 5 > $out/bench_r02_market_n1.json 2> $out/market.err
 python bench.py --workload hard --steps 30 --warmup 5 > $out/bench_r02_hard_n1.json 2> $out/hard.err

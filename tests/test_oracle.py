@@ -126,67 +126,6 @@ def test_cluster_memory_oracle_matches_reference(path):
     np.testing.assert_allclose(f_hard, g["features_after_hard"], rtol=1e-4, atol=1e-6)
 
 
-def test_infomap_front_end_oracle_matches_reference():
-    """f1: oracle/infomap.py against the unmodified reference functions (infomap_cluster.py get_dist_nbr, get_links)."""
-    from oracle import ref_shim, infomap as oi
-    if not ref_shim.available():
-        pytest.skip("reference tree not present")
-    from reid_gan_b200.synth import synth
-    m = ref_shim.load_infomap_cluster()
-    x, _ = synth(500, 64, 20, 0.8, 3)
-    d_ref, n_ref = m.get_dist_nbr(features=x.numpy(), k=15, knn_method='faiss-cpu')
-    d, n = oi.get_dist_nbr(x.numpy(), 15)
-    assert d.dtype == d_ref.dtype and n.dtype == n_ref.dtype
-    assert np.array_equal(n_ref, n) and np.array_equal(d_ref, d)
-    for min_sim in (0.3, 0.5, 0.9):
-        s_ref, l_ref = m.get_links(single=[], links={}, nbrs=n_ref, dists=d_ref, min_sim=min_sim)
-        s, l = oi.get_links(n, d, min_sim)
-        assert s_ref == s and l_ref == l
-
-
-def test_eval_rerank_oracle_matches_reference():
-    """f2: oracle/eval_rerank.py against the unmodified utils/rerank.py re_ranking."""
-    from oracle import ref_shim, eval_rerank as oe
-    if not ref_shim.available():
-        pytest.skip("reference tree not present")
-    m = ref_shim.load_eval_rerank()
-    qg, qq, gg = oe.synthetic_distances(360, 100, 64, 24, 4)
-    for k1, k2, lam in ((20, 6, 0.3), (7, 1, 0.5), (12, 3, 0.0)):
-        ref = m.re_ranking(qg, qq, gg, k1=k1, k2=k2, lambda_value=lam)
-        got = oe.re_ranking(qg, qq, gg, k1, k2, lam)
-        assert got.dtype == ref.dtype and got.shape == ref.shape
-        assert np.abs(ref - got).max() <= 1e-6
-
-
-def _eval_set(N, Q, D, n_ids, seed, n_cams=4):
-    from reid_gan_b200.synth import synth
-    x, ids = synth(N, D, n_ids, 1.2, seed)
-    cams = np.random.default_rng(seed).integers(0, n_cams, N)
-    return (x[:Q].numpy(), x[Q:].numpy(), ids[:Q].numpy(), ids[Q:].numpy(), cams[:Q], cams[Q:])
-
-
-def test_ranking_oracle_matches_reference():
-    """f3: oracle/ranking.py against the unmodified evaluation_metrics/ranking.py and evaluators.pairwise_distance."""
-    import torch
-    from oracle import ref_shim, ranking as orank
-    if not ref_shim.available():
-        pytest.skip("reference tree not present")
-    m = ref_shim.load_ranking()
-    q, g, qi, gi, qc, gc = _eval_set(600, 130, 32, 28, 5)
-    xx, yy = torch.from_numpy(q), torch.from_numpy(g)
-    dm = torch.pow(xx, 2).sum(1, keepdim=True).expand(len(q), len(g)) + torch.pow(yy, 2).sum(1, keepdim=True).expand(len(g), len(q)).t()
-    dm = dm.clone()
-    dm.addmm_(xx, yy.t(), beta=1, alpha=-2)                    # evaluators.py:84-86
-    assert np.abs(orank.pairwise_distance(q, g) - dm.numpy()).max() <= 2e-6
-    assert abs(m.mean_ap(dm, qi, gi, qc, gc) - orank.mean_ap(dm.numpy(), qi, gi, qc, gc)) <= 1e-12
-    for kw in (dict(first_match_break=True), dict(), dict(separate_camera_set=True, first_match_break=True)):
-        a = m.cmc(dm, qi, gi, qc, gc, topk=30, single_gallery_shot=False, **kw)
-        b = orank.cmc(dm.numpy(), qi, gi, qc, gc, topk=30, **kw)
-        assert np.abs(a - b).max() <= 1e-12
-    # defaults (ids = arange, cameras 0 / 1)
-    assert abs(m.mean_ap(dm[:, :130]) - orank.mean_ap(dm.numpy()[:, :130])) <= 1e-12
-
-
 # ---- golden vectors of the "next" rows (generated by oracle/make_golden.py from the unmodified reference) ----
 def _gold(name):
     return np.load(os.path.join(GOLD, name))
