@@ -478,6 +478,18 @@ int reid_cm_grad_inputs(const float* g, const float* centroids, int64_t B, int64
  * workspace: B int32. */
 int reid_cm_update(const float* xhat, const int64_t* targets, float* centroids, int64_t B, int64_t C,
                    int64_t D, float momentum, int hard, void* workspace, void* stream);
+/* One ClusterMemory over `world` ranks (DistributedClusterMemory; the reference's nn.DataParallel gathers every GPU's
+ * batch onto one memory, train_usl.py:189): reid_cm_forward on this rank's B rows, and the same CTA that writes row b's
+ * xhat also stores it, with the row's target, into slot me * cap + b of EVERY rank's receive buffer.  peer_base[w]
+ * (device array of `world` addresses) is rank w's buffer: world * cap int64 targets, then world * cap x D fp32 xhat.
+ * Slots B <= b < cap of this rank get target -1.  After a barrier across the ranks, reid_cm_update on the local
+ * buffer (B = world * cap rows) applies the update of the concatenated batch in rank order; the padding rows are
+ * skipped.  The split-K count is that of B_split rows (pass world * cap): z, loss and the gradients then equal the
+ * single-process values of the concatenated batch.  B <= cap, B <= B_split, D <= 4096.
+ * scratch: reid_cm_forward_scratch_bytes(B_split, C, D) bytes. */
+int reid_cm_forward_push(const float* inputs, const int64_t* targets, const float* centroids, int64_t B, int64_t C,
+                         int64_t D, float temp, int64_t B_split, float* loss, float* xhat, float* inv_norm, float* z,
+                         void* scratch, int me, int world, int64_t cap, const uint64_t* peer_base, void* stream);
 
 #ifdef __cplusplus
 }

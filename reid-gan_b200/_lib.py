@@ -98,6 +98,7 @@ SIGNATURES = {
     "reid_cm_logits": (_I, [_P, _P, _L, _L, _L, _P, _P]),
     "reid_cm_grad_inputs": (_I, [_P, _P, _L, _L, _L, _P, _P]),
     "reid_cm_update": (_I, [_P, _P, _P, _L, _L, _L, _F, _I, _P, _P]),
+    "reid_cm_forward_push": (_I, [_P, _P, _P, _L, _L, _L, _F, _L, _P, _P, _P, _P, _P, _I, _I, _L, _P, _P]),
 }
 
 _lib = None

@@ -129,20 +129,40 @@ __device__ __forceinline__ float block_max(float v, float* red) {
 }
 
 // One CTA per sample: ||x||, xhat, z = (sum of split-K partials) / (||x|| * temp), loss.
+// kPush (reid_cm_forward_push): the CTA also stores the row's target and xhat into slot me * cap + b of EVERY rank's
+// receive buffer (peer_base[w]: W * cap int64 targets, then W * cap x D fp32 xhat).  The grid then covers cap rows:
+// the CTAs of rows B <= b < cap only store target -1 (the update kernel skips it).
+template <bool kPush>
 __global__ void __launch_bounds__(256) cm_loss_kernel(const float* __restrict__ inputs,
                                                       const int64_t* __restrict__ targets,
                                                       const float* __restrict__ partial, int splits, int64_t B,
                                                       int64_t C, int64_t D, float temp, float* __restrict__ loss,
                                                       float* __restrict__ xhat, float* __restrict__ inv_norm,
-                                                      float* __restrict__ z) {
+                                                      float* __restrict__ z, int me, int W, int64_t cap,
+                                                      const unsigned long long* __restrict__ peer_base) {
   __shared__ float red[8];
   const int64_t b = blockIdx.x;
+  const int64_t slot = (int64_t)me * cap + b;
+  if (kPush) {
+    for (int w = threadIdx.x; w < W; w += blockDim.x)
+      reinterpret_cast<int64_t*>(peer_base[w])[slot] = b < B ? targets[b] : -1;
+    if (b >= B) {
+      __threadfence_system();
+      return;
+    }
+  }
   const float* x = inputs + b * D;
   float ss = 0.f;
   for (int64_t d = threadIdx.x; d < D; d += blockDim.x) ss = fmaf(x[d], x[d], ss);
   ss = block_sum(ss, red);
   const float inv = 1.0f / fmaxf(sqrtf(ss), 1e-12f);  // F.normalize(eps=1e-12), cm.py:125
-  for (int64_t d = threadIdx.x; d < D; d += blockDim.x) xhat[b * D + d] = x[d] * inv;
+  for (int64_t d = threadIdx.x; d < D; d += blockDim.x) {
+    const float v = x[d] * inv;
+    xhat[b * D + d] = v;
+    if (kPush)
+      for (int w = 0; w < W; ++w)
+        reinterpret_cast<float*>(reinterpret_cast<int64_t*>(peer_base[w]) + (int64_t)W * cap)[slot * D + d] = v;
+  }
   if (threadIdx.x == 0) inv_norm[b] = inv;
   const float scale = inv / temp;
   float mx = -INFINITY;
@@ -163,6 +183,7 @@ __global__ void __launch_bounds__(256) cm_loss_kernel(const float* __restrict__ 
     const int64_t y = targets[b];
     loss[b] = (y >= 0 && y < C) ? (mx + logf(se)) - z[b * C + y] : __int_as_float(0x7fc00000);
   }
+  if (kPush) __threadfence_system();
 }
 
 // gz[b][c] = (softmax(z_b)[c] - [c == y_b]) * grad_loss[b] / temp
@@ -330,7 +351,32 @@ int reid_cm_forward(const float* inputs, const int64_t* targets, const float* ce
   float* partial = (float*)scratch;
   int rc = launch_gemm(true, inputs, centroids, B, C, D, splits, partial, st);
   if (rc != REID_OK) return rc;
-  cm_loss_kernel<<<(unsigned)B, 256, 0, st>>>(inputs, targets, partial, splits, B, C, D, temp, loss, xhat, inv_norm, z);
+  cm_loss_kernel<false><<<(unsigned)B, 256, 0, st>>>(inputs, targets, partial, splits, B, C, D, temp, loss, xhat,
+                                                      inv_norm, z, 0, 1, 0, nullptr);
+  REID_LAUNCH_CHECK();
+  return REID_OK;
+}
+
+int reid_cm_forward_push(const float* inputs, const int64_t* targets, const float* centroids, int64_t B, int64_t C,
+                         int64_t D, float temp, int64_t B_split, float* loss, float* xhat, float* inv_norm, float* z,
+                         void* scratch, int me, int world, int64_t cap, const uint64_t* peer_base, void* stream) {
+  using namespace reid;
+  REID_CHECK_ARG(inputs && targets && centroids && loss && xhat && inv_norm && z && scratch && peer_base,
+                 "reid_cm_forward_push: NULL pointer");
+  REID_CHECK_ARG(B > 0 && C > 0 && D > 0 && temp > 0.f, "reid_cm_forward_push: bad shape/temp");
+  REID_CHECK_ARG(world >= 1 && me >= 0 && me < world, "reid_cm_forward_push: bad rank me=%d of world=%d", me, world);
+  REID_CHECK_ARG(B <= cap && B <= B_split, "reid_cm_forward_push: B=%lld exceeds cap=%lld or B_split=%lld",
+                 (long long)B, (long long)cap, (long long)B_split);
+  REID_CHECK_ARG(D <= 256 * kUpdMaxPerThread, "reid_cm_forward_push: D=%lld exceeds %d", (long long)D,
+                 256 * kUpdMaxPerThread);
+  cudaStream_t st = (cudaStream_t)stream;
+  const int splits = pick_splits(B_split, C, D);  // the split-K count of the whole (all-rank) batch
+  float* partial = (float*)scratch;
+  int rc = launch_gemm(true, inputs, centroids, B, C, D, splits, partial, st);
+  if (rc != REID_OK) return rc;
+  cm_loss_kernel<true><<<(unsigned)cap, 256, 0, st>>>(inputs, targets, partial, splits, B, C, D, temp, loss, xhat,
+                                                      inv_norm, z, me, world, cap,
+                                                      (const unsigned long long*)peer_base);
   REID_LAUNCH_CHECK();
   return REID_OK;
 }

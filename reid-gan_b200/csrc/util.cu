@@ -202,7 +202,7 @@ static int scan_state_for(cudaStream_t stream, size_t n_tiles, ScanState** out) 
 
 extern "C" {
 
-int reid_abi_version(void) { return 4; }
+int reid_abi_version(void) { return 5; }
 const char* reid_last_error(void) { return reid::g_err; }
 uint64_t reid_launch_count(void) { return reid::g_launches; }
 
