@@ -392,6 +392,42 @@ int reid_rr_weights(const float* dist, int64_t M, const int32_t* E_pad, int stri
                     int64_t n_rows, int32_t* E_idx, float* V_val, void* stream);
 int reid_rr_final(const float* J, int64_t ldJ, const float* dist, int64_t Q, int64_t G, float one_minus_lambda,
                   float lambda, float* out, void* stream);
+
+/* ---- f2 from features (re_ranking_features): the same result from the (M x D) union x = [query; gallery] ----
+ * Nothing of M^2 elements exists.  With orig(r, c) = sq(r, c)^2 and colmax[c] = max_r orig(r, c), dist[i, j] =
+ * orig(j, i) / colmax[i]: the neighbour lists are the squared-L2 kNN of x (reid_knn_*), colmax comes from a
+ * farthest-neighbour search, the weights and the blend read gathered feature rows and the Q x G distance block.
+ * Distance arithmetic of these entries: sqnorm[i] = sum_d x[i,d]^2 and the dot x_i.x_j accumulated in fp64 (one fixed
+ * order, so sq(i, j) and sq(j, i) have the same bits), sq(i, j) = fp32((sqnorm[i] + sqnorm[j]) - 2 x_i.x_j) formed in
+ * fp64, orig = fp32(sq * sq).
+ *   reid_rr_row_sqnorm64     : sqnorm[i] (fp64) for i < n_rows -- the norms the other entries take.
+ *   reid_rr_farthest_certify : colmax of rows [row_begin, row_end) from the candidate lists of
+ *       reid_knn_candidates_tc_ab run with the NEGATED fp16 operand as xb (scores ~ -x_i.x_j; lists row-major,
+ *       n_lists per row, list_cap entries each).  sqnorm_range = { max, min } fp32 squared norms
+ *       (reid_features_to_half) gives the fp16 error bound eps and the norm spread.  With a_max the best listed score,
+ *       the row is certified when no list overflowed and its rejection threshold lies below
+ *       lo = a_max - 2 eps - (max - min) / 2; then the farthest row is among the listed entries >= lo, which are
+ *       re-scored exactly (at most 128; every |approx - exact| is audited against eps).  A certified row gets its
+ *       exact colmax; an uncertified one gets colmax 0, uncertified_flag[row - row_begin] = 1 and
+ *       *uncertified_count += 1 (optional) -- the caller redoes it with reid_rr_farthest_exact.
+ *   reid_rr_farthest_exact   : colmax[row] = max over all M rows of orig(row, j), exact CUDA-core scan, for the rows
+ *       rows[0 .. n_rows) (or row_begin + r when rows is NULL).  D * 4 <= 200 KB.
+ *   reid_rr_weights_features : reid_rr_weights with orig(e, i) / colmax[i] gathered from the feature rows (:66-67).
+ *   reid_rr_final_qg         : rows [row_begin, row_end) of out (Q x G):  J[i - row_begin][Q + g] * (1 - lambda) +
+ *       (q_g[i][g]^2 / colmax[i]) * lambda, fp32 in the reference's order; J holds those rows (leading dimension ldJ),
+ *       q_g is the Q x G block of reid_pairwise_distance. */
+int reid_rr_row_sqnorm64(const float* x, int64_t n_rows, int64_t D, double* sqnorm, void* stream);
+int reid_rr_farthest_certify(const float* x, int64_t M, int64_t D, const double* sqnorm, const uint64_t* cand,
+                             const int32_t* cand_cnt, const uint32_t* row_tau, int n_lists, int list_cap, int64_t row_begin,
+                             int64_t row_end, const float* sqnorm_range, float* colmax, int32_t* uncertified_flag,
+                             uint64_t* uncertified_count, void* stream);
+int reid_rr_farthest_exact(const float* x, int64_t M, int64_t D, const double* sqnorm, const int32_t* rows,
+                           int64_t row_begin, int64_t n_rows, float* colmax, void* stream);
+int reid_rr_weights_features(const float* x, int64_t M, int64_t D, const double* sqnorm, const float* colmax,
+                             const int32_t* E_pad, int stride, const int64_t* E_ptr, int64_t n_rows, int32_t* E_idx,
+                             float* V_val, void* stream);
+int reid_rr_final_qg(const float* J, int64_t ldJ, const float* q_g, const float* colmax, int64_t Q, int64_t G,
+                     int64_t row_begin, int64_t row_end, float one_minus_lambda, float lambda, float* out, void* stream);
 /* exact top-k of every row of a dense (n_rows x N) key matrix: descending (ties by smaller index), or the k
  * smallest in ascending order when `ascending` != 0. */
 int reid_select_rows(const float* keys, int64_t N, int64_t n_rows, int k, int ascending, int32_t* out_idx,

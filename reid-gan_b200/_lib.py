@@ -74,6 +74,11 @@ SIGNATURES = {
     "reid_rr_normalised_distance": (_I, [_P, _P, _P, _L, _L, _P, _P, _P, _P]),
     "reid_rr_weights": (_I, [_P, _L, _P, _I, _P, _L, _P, _P, _P]),
     "reid_rr_final": (_I, [_P, _L, _P, _L, _L, _F, _F, _P, _P]),
+    "reid_rr_row_sqnorm64": (_I, [_P, _L, _L, _P, _P]),
+    "reid_rr_farthest_certify": (_I, [_P, _L, _L, _P, _P, _P, _P, _I, _I, _L, _L, _P, _P, _P, _P, _P]),
+    "reid_rr_farthest_exact": (_I, [_P, _L, _L, _P, _P, _L, _L, _P, _P]),
+    "reid_rr_weights_features": (_I, [_P, _L, _L, _P, _P, _P, _I, _P, _L, _P, _P, _P]),
+    "reid_rr_final_qg": (_I, [_P, _L, _P, _P, _L, _L, _L, _L, _F, _F, _P, _P]),
     "reid_select_rows": (_I, [_P, _L, _L, _I, _I, _P, _P, _P]),
     "reid_pairwise_distance": (_I, [_P, _P, _L, _L, _L, _P, _P, _P]),
     "reid_rank_metrics_smem_bytes": (_Z, [_L]),

@@ -14,6 +14,11 @@ written against the reference's dict keeps working (`features[f]`, iteration, le
 extracts only its contiguous share of the sorted list (`shard_items`) and hands its rows to
 `sharded.pseudo_labels(x_local, N=N)`: collective (1) of SURVEY 8(e), the feature all-gather, then moves fp32 rows over
 NVLink instead of every rank extracting or uploading all N.
+
+`Evaluator` and `evaluate_all` are the drop-ins of the evaluation entry points (evaluators.py:91-142): the features
+stay on the device, the Q x G distance matrix is computed there and scored there, and `rerank=True` re-ranks from the
+features (rerank.re_ranking_features, reusing the Q x G block) -- no Q x Q or G x G matrix and no host copy of any
+distance matrix.
 """
 import time
 from collections import OrderedDict
@@ -153,3 +158,55 @@ def shard_items(sorted_items, group=None, world=None, rank=None):
     n = len(sorted_items)
     r0, r1 = partition(n, world, rank)
     return list(sorted_items[r0:r1]), r0, r1, n
+
+
+def evaluate_all(query_features, gallery_features, distmat, query=None, gallery=None, query_ids=None, gallery_ids=None,
+                 query_cams=None, gallery_cams=None, cmc_topk=(1, 5, 10), cmc_flag=False):
+    """evaluators.py:91-124.  Returns mAP, or (cmc_scores, mAP) with cmc_flag (the 'market1501' CMC configuration).
+    `distmat` may be a CUDA tensor: it is scored where it is."""
+    from .evaluation import cmc, mean_ap
+    if query is not None and gallery is not None:
+        query_ids = [pid for _, pid, _ in query]
+        gallery_ids = [pid for _, pid, _ in gallery]
+        query_cams = [cam for _, _, cam in query]
+        gallery_cams = [cam for _, _, cam in gallery]
+    else:
+        assert (query_ids is not None and gallery_ids is not None
+                and query_cams is not None and gallery_cams is not None)
+    mAP = mean_ap(distmat, query_ids, gallery_ids, query_cams, gallery_cams)
+    print('Mean AP: {:4.1%}'.format(mAP))
+    if not cmc_flag:
+        return mAP
+    cmc_configs = {
+        'market1501': dict(separate_camera_set=False, single_gallery_shot=False, first_match_break=True)}
+    cmc_scores = {name: cmc(distmat, query_ids, gallery_ids, query_cams, gallery_cams, **params)
+                  for name, params in cmc_configs.items()}
+    print('CMC Scores:')
+    for k in cmc_topk:
+        print('  top-{:<4}{:12.1%}'.format(k, cmc_scores['market1501'][k - 1]))
+    return cmc_scores['market1501'], mAP
+
+
+class Evaluator(object):
+    """evaluators.py:127-142 on the device: one gather each for the query and gallery rows of the extracted features,
+    the Q x G distances on the device, metrics on the device; rerank=True re-ranks from the features."""
+
+    def __init__(self, model):
+        super(Evaluator, self).__init__()
+        self.model = model
+
+    def evaluate(self, data_loader, query, gallery, cmc_flag=False, rerank=False):
+        from .evaluation import pairwise_distance_device
+        from .rerank import _re_ranking_features
+        features, _ = extract_features(self.model, data_loader)
+        dev = features.device
+        with torch.cuda.device(dev), torch.no_grad():
+            query_features = features.matrix([f for f, _, _ in query])
+            gallery_features = features.matrix([f for f, _, _ in gallery])
+            distmat = pairwise_distance_device(query_features, gallery_features)
+        results = evaluate_all(query_features, gallery_features, distmat, query=query, gallery=gallery, cmc_flag=cmc_flag)
+        if not rerank:
+            return results
+        print('Applying person re-ranking ...')
+        distmat, _ = _re_ranking_features(query_features, gallery_features, q_g_dist=distmat)
+        return evaluate_all(query_features, gallery_features, distmat, query=query, gallery=gallery, cmc_flag=cmc_flag)
