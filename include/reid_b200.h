@@ -449,6 +449,9 @@ int reid_rank_metrics(const float* dist, int64_t m, int64_t n, int64_t ld, const
                       const int64_t* q_cams, const int64_t* g_cams, int separate_camera_set, int topk,
                       int first_match_break, double* ap_out, int32_t* has_pos, double* cmc_contrib, double* cmc_ret,
                       void* stream);
+/* cmc_ret[k] = sum over i = 0..m-1, in order, of cmc_contrib[i * topk + k]: the reduction reid_rank_metrics runs, on
+ * contributions gathered from several ranks (distributed evaluation), so the sum has the single-process order. */
+int reid_cmc_reduce(const double* cmc_contrib, int64_t m, int topk, double* cmc_ret, void* stream);
 
 /* ---- a9: centroid init  (train_usl.py:169-182, 191) -------------------------------
  * out[k] = mean of x[i] over labels[i] == k, k = 0..C-1 (labels < 0 skipped), members added in
@@ -485,6 +488,13 @@ int reid_peer_push_records(const int32_t* cnt, const int64_t* ptr, const int32_t
                            int64_t rec_offset_bytes, void* stream);
 int reid_peer_allgather(const void* src, int64_t block_bytes, int me, int world, const uint64_t* peer_base,
                         int64_t dst_offset_bytes, void* stream);
+/* reid_peer_scatter_rows: the feature exchange of distributed evaluation.  src: this rank's n_rows extracted feature
+ * rows (D floats each, D % 4 == 0, 16-byte aligned).  Local row r is stored as rows dst_rows[2r] and dst_rows[2r + 1]
+ * (-1: not in that list) of the (M, D) fp32 matrix [query; gallery] at peer_base[w] + dst_offset_bytes, for every
+ * w < world -- a file name in both lists is written twice.  A destination >= M is never written; bad_count (optional
+ * device uint64) counts them.  With world = 1 and a local base it is a plain scatter (the collective fallback). */
+int reid_peer_scatter_rows(const float* src, int64_t n_rows, int64_t D, const int32_t* dst_rows, int64_t M, int world,
+                           const uint64_t* peer_base, int64_t dst_offset_bytes, uint64_t* bad_count, void* stream);
 
 /* ---- f4: feature hand-off  (clustercontrast/evaluators.py:16-68, train_usl.py:152-153) ----------------
  * dst[r] = src[idx[r]] for r < n (rows of D floats, D % 4 == 0): re-orders a device-resident feature store into the

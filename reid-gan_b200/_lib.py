@@ -95,6 +95,8 @@ SIGNATURES = {
     "reid_peer_push_lists": (_I, [_P, _P, _I, _L, _I, _I, _P, _L, _P]),
     "reid_peer_push_records": (_I, [_P, _P, _P, _P, _L, _L, _I, _I, _I, _P, _L, _P]),
     "reid_peer_allgather": (_I, [_P, _L, _I, _I, _P, _L, _P]),
+    "reid_peer_scatter_rows": (_I, [_P, _L, _L, _P, _L, _I, _P, _L, _P, _P]),
+    "reid_cmc_reduce": (_I, [_P, _L, _I, _P, _P]),
     "reid_gather_rows": (_I, [_P, _L, _P, _L, _L, _P, _P]),
     "reid_centroids_dev": (_I, [_P, _L, _L, _P, _P, _L, _I, _P, _P, _P]),
     "reid_cm_forward_scratch_bytes": (_Z, [_L, _L, _L]),

@@ -268,4 +268,12 @@ int reid_rank_metrics(const float* dist, int64_t m, int64_t n, int64_t ld, const
   }
   return REID_OK;
 }
+
+int reid_cmc_reduce(const double* cmc_contrib, int64_t m, int topk, double* cmc_ret, void* stream) {
+  using namespace reid;
+  REID_CHECK_ARG(cmc_contrib && cmc_ret && m >= 1 && topk >= 1, "reid_cmc_reduce: bad arguments");
+  cmc_reduce_kernel<<<(unsigned)((topk + 127) / 128), 128, 0, (cudaStream_t)stream>>>(cmc_contrib, m, topk, cmc_ret);
+  REID_LAUNCH_CHECK();
+  return REID_OK;
+}
 }

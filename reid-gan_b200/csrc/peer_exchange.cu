@@ -80,6 +80,36 @@ __global__ void __launch_bounds__(256) peer_allgather_kernel(const uint32_t* __r
   __threadfence_system();
 }
 
+// reid_peer_scatter_rows: the feature all-gather of distributed evaluation.  Local row r goes to rows dst[2r] and
+// dst[2r + 1] of the (M, D) matrix [query; gallery] of every rank (-1: not in that list).  One warp per row: each
+// float4 of the row is loaded once and stored 2 x W times.  A destination >= M is counted and never written.
+__global__ void __launch_bounds__(256) peer_scatter_rows_kernel(const float4* __restrict__ src, int64_t n_rows, int64_t D4,
+                                                                const int32_t* __restrict__ dst_rows, int64_t M, int W,
+                                                                const unsigned long long* __restrict__ peer_base,
+                                                                int64_t dst_offset_bytes,
+                                                                unsigned long long* __restrict__ bad_count) {
+  const int64_t row = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (row >= n_rows) return;
+  const int lane = lane_id();
+  int64_t d0 = dst_rows[2 * row], d1 = dst_rows[2 * row + 1];
+  if (d0 >= M || d1 >= M) {
+    if (lane == 0 && bad_count) atomicAdd(bad_count, (unsigned long long)((d0 >= M) + (d1 >= M)));
+    if (d0 >= M) d0 = -1;
+    if (d1 >= M) d1 = -1;
+  }
+  if (d0 < 0 && d1 < 0) return;
+  const float4* s = src + row * D4;
+  for (int64_t c = lane; c < D4; c += 32) {
+    const float4 v = s[c];
+    for (int w = 0; w < W; ++w) {
+      float4* x = reinterpret_cast<float4*>(reinterpret_cast<unsigned char*>(peer_base[w]) + dst_offset_bytes);
+      if (d0 >= 0) x[d0 * D4 + c] = v;
+      if (d1 >= 0) x[d1 * D4 + c] = v;
+    }
+  }
+  __threadfence_system();
+}
+
 }  // namespace reid
 
 extern "C" {
@@ -129,6 +159,24 @@ int reid_peer_allgather(const void* src, int64_t block_bytes, int me, int world,
   peer_allgather_kernel<<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>((const uint32_t*)src, n4, me, world,
                                                                          (const unsigned long long*)peer_base,
                                                                          dst_offset_bytes);
+  REID_LAUNCH_CHECK();
+  return REID_OK;
+}
+
+int reid_peer_scatter_rows(const float* src, int64_t n_rows, int64_t D, const int32_t* dst_rows, int64_t M, int world,
+                           const uint64_t* peer_base, int64_t dst_offset_bytes, uint64_t* bad_count, void* stream) {
+  using namespace reid;
+  REID_CHECK_ARG(n_rows == 0 || (src && dst_rows), "reid_peer_scatter_rows: NULL pointer");
+  REID_CHECK_ARG(peer_base && n_rows >= 0 && M >= 1 && world >= 1 && D >= 1 && dst_offset_bytes >= 0,
+                 "reid_peer_scatter_rows: bad arguments");
+  REID_CHECK_ARG(D % 4 == 0, "reid_peer_scatter_rows: D=%lld is not a multiple of 4", (long long)D);
+  REID_CHECK_ARG(((uintptr_t)src & 15) == 0 && dst_offset_bytes % 16 == 0,
+                 "reid_peer_scatter_rows: src and dst_offset_bytes must be 16-byte aligned");
+  if (n_rows == 0) return REID_OK;
+  REID_CHECK_ARG((n_rows + 7) / 8 < (1LL << 31), "reid_peer_scatter_rows: too many rows");
+  peer_scatter_rows_kernel<<<(unsigned)((n_rows + 7) / 8), 256, 0, (cudaStream_t)stream>>>(
+      (const float4*)src, n_rows, D / 4, dst_rows, M, world, (const unsigned long long*)peer_base, dst_offset_bytes,
+      (unsigned long long*)bad_count);
   REID_LAUNCH_CHECK();
   return REID_OK;
 }

@@ -160,6 +160,22 @@ def shard_items(sorted_items, group=None, world=None, rank=None):
     return list(sorted_items[r0:r1]), r0, r1, n
 
 
+def eval_shard(query, gallery, group=None, world=None, rank=None):
+    """This rank's share of the test images for DistributedEvaluator: the union of `query` and `gallery` (items
+    (fname, pid, cam); a file name in both lists counts once), sorted by file name, split into the contiguous blocks
+    of sharded.partition.  Build the rank's test loader over these items."""
+    from .sharded import partition
+    if world is None:
+        import torch.distributed as dist
+        world, rank = dist.get_world_size(group), dist.get_rank(group)
+    union = {}
+    for item in list(query) + list(gallery):
+        union.setdefault(item[0], item)
+    names = sorted(union)
+    r0, r1 = partition(len(names), world, rank)
+    return [union[f] for f in names[r0:r1]]
+
+
 def evaluate_all(query_features, gallery_features, distmat, query=None, gallery=None, query_ids=None, gallery_ids=None,
                  query_cams=None, gallery_cams=None, cmc_topk=(1, 5, 10), cmc_flag=False):
     """evaluators.py:91-124.  Returns mAP, or (cmc_scores, mAP) with cmc_flag (the 'market1501' CMC configuration).
@@ -181,10 +197,14 @@ def evaluate_all(query_features, gallery_features, distmat, query=None, gallery=
         'market1501': dict(separate_camera_set=False, single_gallery_shot=False, first_match_break=True)}
     cmc_scores = {name: cmc(distmat, query_ids, gallery_ids, query_cams, gallery_cams, **params)
                   for name, params in cmc_configs.items()}
+    _print_cmc(cmc_scores['market1501'], cmc_topk)
+    return cmc_scores['market1501'], mAP
+
+
+def _print_cmc(cmc_scores, cmc_topk):
     print('CMC Scores:')
     for k in cmc_topk:
-        print('  top-{:<4}{:12.1%}'.format(k, cmc_scores['market1501'][k - 1]))
-    return cmc_scores['market1501'], mAP
+        print('  top-{:<4}{:12.1%}'.format(k, cmc_scores[k - 1]))
 
 
 class Evaluator(object):

@@ -91,16 +91,17 @@ def _sparse_stages(rank, M, k1, k2, weights, dev):
     return dict(Q=(q_ptr, q_idx, q_val), C=(c_ptr, c_idx, c_val), E=(e_ptr, e_idx[:e_total], v_val[:e_total]))
 
 
-def _jaccard_blend(sparse, M, Q, lambda_value, blend, dev):
-    """rerank.py:80-96: Jaccard rows of the queries in blocks of rows (<= 512 MB each); `blend(J, r0, r1, 1 - lambda,
-    lambda)` writes rows [r0, r1) of the result."""
+def _jaccard_blend(sparse, M, Q, lambda_value, blend, dev, q0=0):
+    """rerank.py:80-96: Jaccard rows of the queries q0..Q-1 in blocks of rows (<= 512 MB each); `blend(J, r0, r1,
+    1 - lambda, lambda)` writes rows [r0, r1) of the result.  Every row is computed on its own: any q0 gives the rows
+    of q0 = 0."""
     sp = stream_ptr()
     q_ptr, q_idx, q_val = sparse["Q"]
     c_ptr, c_idx, c_val = sparse["C"]
-    block = max(1, min(Q, (512 << 20) // (4 * M)))
+    block = max(1, min(Q - q0, (512 << 20) // (4 * M)))
     a_ = float(np.float32(1 - lambda_value))
     b_ = float(np.float32(lambda_value))
-    for r0 in range(0, Q, block):
+    for r0 in range(q0, Q, block):
         r1 = min(Q, r0 + block)
         J = torch.empty((r1 - r0, M), dtype=torch.float32, device=dev)
         call("reid_jaccard_dense", ptr(q_ptr), ptr(q_idx), ptr(q_val), ptr(c_ptr), ptr(c_idx), ptr(c_val), M, r0, r1, ptr(J),
@@ -147,9 +148,10 @@ FARTHEST_KEEP = 16           # candidates kept per list (per row: 2 x column spl
 FARTHEST_BLOCK = 16384       # rows per candidate pass: their lists take 2 x splits x 512 x 8 B = 8..32 KB a row
 
 
-def farthest_colmax(x, sqnorm=None, mode="auto"):
+def farthest_colmax(x, sqnorm=None, mode="auto", rows=None):
     """colmax[i] = max_j fp32(sq(i, j)^2) over all rows j of the (M, D) float32 CUDA tensor x (rerank.py:41's
-    np.max(original_dist, axis=0) of the union).  Returns (colmax float32 (M,), info).
+    np.max(original_dist, axis=0) of the union).  Returns (colmax float32 (M,), info).  rows=(r0, r1): only those rows,
+    colmax is then (r1 - r0,); every value is exact, so it equals colmax[r0:r1] of the whole search bit for bit.
 
     mode "tc" (what "auto" picks for M >= FARTHEST_TC_MIN, D % 64 == 0 and rows of one norm): the fp16 tcgen05 candidate
     kernel of the kNN search run against the NEGATED operand keeps the few smallest approximate dot products per row;
@@ -166,7 +168,8 @@ def farthest_colmax(x, sqnorm=None, mode="auto"):
     if sqnorm is None:
         sqnorm = torch.empty(M, dtype=torch.float64, device=dev)
         call("reid_rr_row_sqnorm64", ptr(x), M, D, ptr(sqnorm), sp)
-    colmax = torch.empty(M, dtype=torch.float32, device=dev)
+    r0, r1 = (0, M) if rows is None else rows
+    colmax = torch.empty(M, dtype=torch.float32, device=dev)          # indexed by global row
     info = {"mode": mode, "uncertified_rows": 0}
     if mode not in ("auto", "tc", "exact"):
         raise ValueError("unknown farthest-search mode %r" % (mode,))
@@ -181,30 +184,30 @@ def farthest_colmax(x, sqnorm=None, mode="auto"):
             del xh
     info["mode"] = mode
     if mode == "exact":
-        call("reid_rr_farthest_exact", ptr(x), M, D, ptr(sqnorm), None, 0, M, ptr(colmax), sp)
-        return colmax, info
+        call("reid_rr_farthest_exact", ptr(x), M, D, ptr(sqnorm), None, r0, r1 - r0, ptr(colmax), sp)
+        return colmax[r0:r1], info
     xn = torch.neg(xh)
-    flag = torch.empty(M, dtype=torch.int32, device=dev)
-    for r0 in range(0, M, FARTHEST_BLOCK):
-        r1 = min(M, r0 + FARTHEST_BLOCK)
-        n = r1 - r0
+    flag = torch.empty(r1 - r0, dtype=torch.int32, device=dev)
+    for b0 in range(r0, r1, FARTHEST_BLOCK):
+        b1 = min(r1, b0 + FARTHEST_BLOCK)
+        n = b1 - b0
         s = ctypes.c_int(1)
         call("reid_knn_tc_plan", M, n, CTA_GROUP, ctypes.byref(s))
         n_lists = 2 * s.value
         cand = torch.empty(n * n_lists * TC_CAP, dtype=torch.int64, device=dev)
         cand_cnt = torch.zeros(n * n_lists, dtype=torch.int32, device=dev)
         tau = torch.empty(n, dtype=torch.int32, device=dev)
-        call("reid_knn_candidates_tc_ab", ptr(xh), M, ptr(xn), M, D, SCALE_LOG2, r0, r1, FARTHEST_KEEP, s.value, CTA_GROUP,
+        call("reid_knn_candidates_tc_ab", ptr(xh), M, ptr(xn), M, D, SCALE_LOG2, b0, b1, FARTHEST_KEEP, s.value, CTA_GROUP,
              ptr(cand), ptr(cand_cnt), ptr(tau), sp)
-        call("reid_rr_farthest_certify", ptr(x), M, D, ptr(sqnorm), ptr(cand), ptr(cand_cnt), ptr(tau), n_lists, TC_CAP, r0, r1,
-             ptr(msq), ptr(colmax), ptr(flag[r0:]), None, sp)
+        call("reid_rr_farthest_certify", ptr(x), M, D, ptr(sqnorm), ptr(cand), ptr(cand_cnt), ptr(tau), n_lists, TC_CAP, b0, b1,
+             ptr(msq), ptr(colmax), ptr(flag[b0 - r0:]), None, sp)
         del cand, cand_cnt, tau
     del xh, xn
-    bad = torch.nonzero(flag).flatten().to(torch.int32).contiguous()
+    bad = (torch.nonzero(flag).flatten() + r0).to(torch.int32).contiguous()
     if bad.numel():
         call("reid_rr_farthest_exact", ptr(x), M, D, ptr(sqnorm), ptr(bad), 0, bad.numel(), ptr(colmax), sp)
     info["uncertified_rows"] = int(bad.numel())
-    return colmax, info
+    return colmax[r0:r1], info
 
 
 def _as_features(a, dev, what):
@@ -218,7 +221,6 @@ def _as_features(a, dev, what):
 def _re_ranking_features(query_features, gallery_features, k1=20, k2=6, lambda_value=0.3, q_g_dist=None):
     """re_ranking_features on the device; returns (out (Q, G) CUDA tensor, parts).  q_g_dist: the (Q, G)
     pairwise_distance_device(q, g) block when the caller has it already (Evaluator.evaluate), else it is computed."""
-    from .evaluation import pairwise_distance_device
     _lib.lib()
     _check_k(k1, k2, 64)                                      # k1 + 1 <= 64 before anything touches a device
     ref = query_features if isinstance(query_features, torch.Tensor) else None
@@ -244,23 +246,45 @@ def _re_ranking_features(query_features, gallery_features, k1=20, k2=6, lambda_v
         colmax, far_info = farthest_colmax(x, sqnorm)
         # :43  initial_rank[:, :k1+1]: a row of dist is a row of orig over a positive constant -- the squared-L2 kNN
         rank, _, knn_info = knn_search(x, cols, "auto")
-
-        def weights(e_pad, e_stride, e_ptr, e_idx, v_val):
-            call("reid_rr_weights_features", ptr(x), M, D, ptr(sqnorm), ptr(colmax), ptr(e_pad), e_stride, ptr(e_ptr), M,
-                 ptr(e_idx), ptr(v_val), sp)
-
-        sparse = _sparse_stages(rank, M, k1, k2, weights, dev)
-        if q_g_dist is None:
-            q_g_dist = pairwise_distance_device(x[:Q], g)
         del g
-        out = torch.empty((Q, G), dtype=torch.float32, device=dev)
-
-        def blend(J, r0, r1, a_, b_):
-            call("reid_rr_final_qg", ptr(J), M, ptr(q_g_dist), ptr(colmax), Q, G, r0, r1, a_, b_, ptr(out), sp)
-
-        _jaccard_blend(sparse, M, Q, lambda_value, blend, dev)
+        sparse = _rr_sparse(x, sqnorm, colmax, rank, k1, k2)
+        out = _rr_blend(x, sparse, colmax, Q, lambda_value, q_g_dist)
         parts = dict(rank=rank, colmax=colmax, E=sparse["E"], knn_info=knn_info, farthest_info=far_info)
         return out, parts
+
+
+def _rr_sparse(x, sqnorm, colmax, rank, k1, k2):
+    """The sparse stages of the re-ranking from features, once colmax and the neighbour lists of all M rows are known.
+    Every query's Jaccard row reads the inverted index of all M rows, so distributed evaluation runs them on every rank."""
+    M, D = x.shape
+    sp = stream_ptr()
+
+    def weights(e_pad, e_stride, e_ptr, e_idx, v_val):
+        call("reid_rr_weights_features", ptr(x), M, D, ptr(sqnorm), ptr(colmax), ptr(e_pad), e_stride, ptr(e_ptr), M,
+             ptr(e_idx), ptr(v_val), sp)
+
+    return _sparse_stages(rank, M, k1, k2, weights, x.device)
+
+
+def _rr_blend(x, sparse, colmax, Q, lambda_value, q_g_dist=None, q0=0, q1=None):
+    """Jaccard rows and blend of the query rows [q0, q1) (default: all Q).  q_g_dist: their (q1 - q0, G) distance
+    block, computed when None.  Returns the (q1 - q0, G) re-ranked rows."""
+    from .evaluation import pairwise_distance_device
+    M = x.shape[0]
+    G = M - Q
+    q1 = Q if q1 is None else q1
+    sp = stream_ptr()
+    if q_g_dist is None:
+        q_g_dist = pairwise_distance_device(x[q0:q1], x[Q:])
+    out = torch.empty((q1 - q0, G), dtype=torch.float32, device=x.device)
+    Jq = Q - (q1 - q0)              # rr_final_qg reads J[r, Q + g]: with a (q1 - q0)-row block, shift J by the rows left out
+
+    def blend(J, r0, r1, a_, b_):
+        call("reid_rr_final_qg", ptr(J.view(-1)[Jq:]), M, ptr(q_g_dist), ptr(colmax[q0:]), q1 - q0, G, r0 - q0, r1 - q0,
+             a_, b_, ptr(out), sp)
+
+    _jaccard_blend(sparse, M, q1, lambda_value, blend, x.device, q0)
+    return out
 
 
 def re_ranking_features(query_features, gallery_features, k1=20, k2=6, lambda_value=0.3, return_device=False):
