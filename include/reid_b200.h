@@ -80,6 +80,7 @@ int reid_knn_exact_l2(const float* x, int64_t N, int64_t D, const int32_t* rows_
  * row owns n_lists = 2 * n_splits candidate lists:
  *   cand[((row-row_begin)*n_lists + l)*REID_TC_CAP + p] = (fp32 score bits << 32) | column,
  *   p < cand_cnt[(row-row_begin)*n_lists + l] <= REID_TC_CAP.
+ * A column appears at most once across a row's lists (reid_knn_rescore ranks by counting strictly greater keys).
  * row_tau[row-row_begin] (order-preserving integer image of a float, 0 = none) is the row's final
  * rejection threshold: every column that is in none of the row's lists scored <= that value, and at
  * least `keep` listed columns score >= it.  Scores are approximate (fp16 inputs); see reid_knn_rescore.
@@ -171,7 +172,10 @@ int reid_knn_rescore_mapped(const float* x, int64_t N, int64_t D, int64_t row_be
 
 /* fp32 features -> scaled fp16 operand; max_sqnorm_out (optional, TWO floats) = { max_i ||x_i||^2, min_i ||x_i||^2 }:
  * the maximum scales the fp16 rounding bound  |approx - exact| <= 2^-10 ||x_i|| ||x_j||, the pair tells the caller
- * whether all rows have one norm (inner-product order == the reference's L2 order) or reid_knn_exact_l2 is needed. */
+ * whether all rows have one norm (inner-product order == the reference's L2 order) or reid_knn_exact_l2 is needed.
+ * Limit: a component with |x| * 2^scale_log2 >= 65520 rounds to +-inf in fp16 and no bound holds for its row's scores;
+ * the maximum is then reported as +inf (no row can be certified), and the minimum stays the true one -- a caller that
+ * needs the true maximum recomputes it with reid_sqnorm_range.  The same holds for _acc and _gather. */
 int reid_features_to_half(const float* x, int64_t n_rows, int64_t D, int scale_log2, void* xh,
                           float* max_sqnorm_out, void* stream);
 /* { 0, 3.4e38 }: the identities of the { max, min } pair, for reid_features_to_half_acc */
@@ -195,6 +199,7 @@ int reid_features_to_half_acc(const float* x, int64_t n_rows, int64_t D, int sca
  * locality_order != 0: the exact stage gathers ~36 feature rows per query row and is HBM bound; rows of one
  * identity cluster share their candidates, so they are visited back to back (counting sort on the smallest
  * index among a row's strong candidates) and repeats become L2 hits.
+ * The lists must be free of duplicates: no column twice across one row's lists.
  * list_cap: entries reserved per list (REID_TC_CAP for reid_knn_candidates_tc, the cap given to
  * reid_knn_candidates_sym); a count above it marks an overflowed list and un-certifies the row.
  * list_pitch_rows: 0 = lists are row-major, list l of local row r at index r * n_lists + l (what the candidate

@@ -437,6 +437,7 @@ __global__ void __launch_bounds__(256) to_half_kernel(const float* __restrict__ 
   for (int64_t row = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); row < n_rows;
        row += (int64_t)gridDim.x * (blockDim.x >> 5)) {
   float ss = 0.f;
+  float amax = 0.f;                                      // largest |x| of the row: an fp16 overflow check
   if ((D & 3) == 0 && ((((uintptr_t)x) | ((uintptr_t)xh)) & 15) == 0) {
     // 16-byte loads, 8-byte stores: the stage is a pure stream (4ND bytes in, 2ND out)
     const int64_t srow = src_row ? (int64_t)src_row[row] : row;      // sample-first layout of the symmetric search
@@ -461,6 +462,7 @@ __global__ void __launch_bounds__(256) to_half_kernel(const float* __restrict__ 
           ss = fmaf(v[u].y, v[u].y, ss);
           ss = fmaf(v[u].z, v[u].z, ss);
           ss = fmaf(v[u].w, v[u].w, ss);
+          amax = fmaxf(amax, fmaxf(fmaxf(fabsf(v[u].x), fabsf(v[u].y)), fmaxf(fabsf(v[u].z), fabsf(v[u].w))));
           const __half2 lo = __floats2half2_rn(v[u].x * scale, v[u].y * scale);
           const __half2 hi = __floats2half2_rn(v[u].z * scale, v[u].w * scale);
           uint2 o;
@@ -474,12 +476,16 @@ __global__ void __launch_bounds__(256) to_half_kernel(const float* __restrict__ 
     for (int64_t d = lane_id(); d < D; d += 32) {
       const float v = x[(src_row ? (int64_t)src_row[row] : row) * D + d];
       ss = fmaf(v, v, ss);
+      amax = fmaxf(amax, fabsf(v));
       xh[row * D + d] = __float2half_rn(v * scale);
     }
   }
   ss = warp_sum(ss);
+  // |x| * 2^s >= 65520 rounds to +-inf in fp16: the row's scores can be inf or NaN (inf - inf) whatever the exact dot,
+  // outside every error bound.  The maximum is then reported as +inf, so eps = inf and no row can be certified.
+  const bool overflow = __any_sync(kFull, !(amax * scale < 65520.f));
   if (lane_id() == 0 && max_sqnorm) {                    // sqnorm_range[0] = max, [1] = min (non-negative floats order like
-    atomicMax((unsigned*)max_sqnorm, __float_as_uint(ss));        // their bit patterns)
+    atomicMax((unsigned*)max_sqnorm, __float_as_uint(overflow ? INFINITY : ss));   // their bit patterns)
     atomicMin((unsigned*)max_sqnorm + 1, __float_as_uint(ss));
   }
   }

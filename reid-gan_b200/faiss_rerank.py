@@ -111,7 +111,7 @@ class RerankState:
             dist.all_reduce(self.report, op=dist.ReduceOp.MAX, group=self._comm.group)
         vals = [int(v) for v in self.report.tolist()]
         self.report, self.report_vals = None, vals
-        if getattr(self, "_check_norms", False) and not _one_norm_info(self.knn_info):
+        if getattr(self, "_check_norms", False) and not _one_norm_info(self.knn_info, self.x):
             st = self._redo("l2")
             self._redo = None
             return (st, False) if check_nbr else st
@@ -143,7 +143,7 @@ def knn_search(x, k, mode="auto", rows=None, defer=False, uncert_count=None, met
     defer: do not read anything back: info["pending"] holds the certificate flags and the repair closure,
     info["max_sqnorm"] the {max, min} squared norms the caller must check (knn_tc.one_norm); uncert_count: device
     scalar that receives the number of uncertified rows."""
-    from .knn_tc import one_norm
+    from .knn_tc import one_norm, sqnorm_range_of
     L = _lib.lib()
     N, D = x.shape
     dev = x.device
@@ -166,7 +166,7 @@ def knn_search(x, k, mode="auto", rows=None, defer=False, uncert_count=None, met
         from .knn_tc import knn_search_tc
         idx, key, info = knn_search_tc(x, k, r0, r1, idx, key, info, defer=defer, uncert_count=uncert_count)
         info["metric"] = "ip"
-        if metric == "auto" and not defer and not one_norm(info["max_sqnorm"].tolist()):
+        if metric == "auto" and not defer and not one_norm(sqnorm_range_of(x, info["max_sqnorm"])):
             _knn_exact_rows(x, k, None, r0, n, idx, key, metric="l2")      # rows of different norms: squared-L2 key
             info.update(mode="exact-l2", metric="l2", visit_order=None, uncertified_rows=0)
         return idx, key, info
@@ -296,7 +296,7 @@ def rerank_state_async(x, k1, k2, knn="auto", rows=None, timers=False, comm=None
         e_cap = max(n, 1) * e_stride                          # upper bound: no size needed on the host
     else:
         vals = report.tolist()                                # read-back 1 of 2: |E| sizes + certificate count
-        if pending is not None and metric == "auto" and not _one_norm_info(info):
+        if pending is not None and metric == "auto" and not _one_norm_info(info, x):
             # rows of different norms: the reference's L2 order is not the inner-product order that was searched
             return rerank_state_async(x, k1, k2, knn="exact", timers=timers, speculative=False, metric="l2", half=half)
         if pending is not None and vals[R_UNCERT]:            # uncertified rows: exact search for them, then redo a2/a3
@@ -429,10 +429,10 @@ def _stride_for(kind, N):
     return max(REC_STRIDE[kind], -(-int(hint * 1.25) // 32) * 32)
 
 
-def _one_norm_info(info):
-    from .knn_tc import one_norm
+def _one_norm_info(info, x):
+    from .knn_tc import one_norm, sqnorm_range_of
     rng = info.get("max_sqnorm")
-    return True if rng is None else one_norm(rng.tolist())
+    return True if rng is None else one_norm(sqnorm_range_of(x, rng))
 
 
 def rank_digest(st):

@@ -32,6 +32,18 @@ def one_norm(sqnorm_range):
     return mx <= mn * (1.0 + UNIT_NORM_TOL)
 
 
+def sqnorm_range_of(x, sqnorm_range):
+    """[max, min] squared norms of the rows of x, from the range reid_features_to_half reported.  That maximum is +inf
+    when a feature overflowed the fp16 operand (|x| * 2^SCALE_LOG2 >= 65520; it makes eps infinite, so no row is
+    certified); the true range is then computed again, so that an overflow alone never picks the squared-L2 key."""
+    rng = sqnorm_range.tolist()
+    if rng[0] == float("inf"):
+        r = torch.empty(2, dtype=torch.float32, device=x.device)
+        call("reid_sqnorm_range", ptr(x), x.shape[0], x.shape[1], ptr(r), stream_ptr())
+        rng = r.tolist()
+    return rng
+
+
 def new_sqnorm_range(dev):
     """{max, min} accumulator for reid_features_to_half_acc: identities {0, 3.4e38}."""
     r = torch.empty(2, dtype=torch.float32, device=dev)

@@ -407,7 +407,7 @@ def knn_search_tiles(x, k, group=None, report=None):
         if report is None:
             bad = torch.nonzero(flag).flatten().to(torch.int32)
             n_bad = bad.numel()
-            if not kt.one_norm(msq.tolist()):              # rows of different norms (every rank sees the same features):
+            if not kt.one_norm(kt.sqnorm_range_of(x, msq)):  # rows of different norms (every rank sees the same features):
                 metric = "l2"                              # the reference's L2 order needs the squared-L2 key
                 _knn_exact_rows(x, k, None, b0, nb, idx[:nb], key[:nb], metric="l2")
                 n_bad = 0
@@ -418,7 +418,7 @@ def knn_search_tiles(x, k, group=None, report=None):
                 _knn_exact_rows(x, k, rows, 0, n_bad, bi, bk)
                 idx[bad.long()] = bi
                 key[bad.long()] = bk
-    elif report is None and not kt.one_norm(msq.tolist()):
+    elif report is None and not kt.one_norm(kt.sqnorm_range_of(x, msq)):
         metric = "l2"
     mark("rescore")
     # 5. final lists of all rows on every rank
