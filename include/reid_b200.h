@@ -137,9 +137,10 @@ int reid_knn_sample_tau(const uint64_t* cand, const int32_t* cand_cnt, const uin
 
 /* ---- sample-first layout of the symmetric search (knn_tc._candidates_sym_sf; replaces the same lines,
  * utils/faiss_rerank.py:39-62).  The fp16 operand is written with the threshold sample in its first m rows
- * (reid_features_to_half_gather), so the prepass -- all rows against rows [0, m) -- computes scores the symmetric
- * pass needs anyway: the prepass hands them to the main lists in both directions and the symmetric pass runs
- * only the tiles (I, J) with m / 256 <= I <= J (12 % fewer tcgen05 tiles at N = 32,621, m = 2,048).
+ * (reid_features_to_half_gather), and the block column [0, m) of the matrix -- all rows against the sample --
+ * gives both the thresholds and candidates the symmetric pass needs: it is scored once, its scores go to the main
+ * lists in both directions, and the symmetric pass runs only the tiles (I, J) with m / 256 <= I <= J (12 % fewer
+ * tcgen05 tiles at N = 32,621, m = 2,048).  The sample rows against the sample run through the prepass entries:
  *   reid_knn_candidates_tc_abt : reid_knn_candidates_tc_ab + the transposed direction -- tau_col[j] is the (already
  *       known) threshold of column row j; every score above it is appended to cand_col[j * cap_col + ..] with the
  *       query row as its column (tau_col = NULL: off); publish_final: row_tau additionally receives every list's final
@@ -151,7 +152,18 @@ int reid_knn_sample_tau(const uint64_t* cand, const int32_t* cand_cnt, const uin
  *       threshold when fewer than r scores are listed above the floor;
  *   reid_knn_rescore_mapped    : reid_knn_rescore on lists that live in the permuted row space -- row r's lists and
  *       threshold are those of position row_pos[r], a listed column p is the original row col_orig[p] (both NULL:
- *       plain reid_knn_rescore). */
+ *       plain reid_knn_rescore).
+ * The other rows against the sample run on the symmetric kernel with a provisional threshold: a row only needs a
+ * threshold that every unlisted column scored at or below, and a lower one only lengthens its list:
+ *   reid_knn_tau_floor         : tau' = the smallest of the sample rows' thresholds tau_ord[0, m), written to tau[m, N)
+ *       and tau_ord[m, N) -- on the device, no host round trip;
+ *   reid_knn_candidates_sym_tiles : reid_knn_candidates_sym, for the tiles (I, J) with I < m / 256 <= J: sample row i
+ *       lists column j above tau[i], row j lists sample column i above tau[j] = tau'.  A separate entry so that the
+ *       per-entry timings keep the block column apart from the symmetric pass over the other tiles;
+ *   reid_knn_list_tau          : for rows [row0, row0 + n_rows) whose list holds exactly their scores above tau_ord[row]
+ *       (here: the sample scores above tau'), raise tau[row] / tau_ord[row] to the r-th best listed score (its top 16
+ *       bits, rounded down) when at least r are listed and it is higher; otherwise tau' stays.  Only the first
+ *       min(cand_cnt[row], cap, 1024) entries are read (a subset can only lower the result). */
 /* xh[i] = fp16(2^s x[src_row[i]]), i < n_rows; max_sqnorm_inout accumulates like reid_features_to_half_acc */
 int reid_features_to_half_gather(const float* x, const int32_t* src_row, int64_t n_rows, int64_t D, int scale_log2,
                                  void* xh, float* max_sqnorm_inout, void* stream);
@@ -169,6 +181,12 @@ int reid_knn_rescore_mapped(const float* x, int64_t N, int64_t D, int64_t row_be
                             int locality_order, const int32_t* row_pos, const int32_t* col_orig, int32_t* out_idx,
                             float* out_key, int32_t* uncertified_flag, float* max_err_out, void* workspace,
                             uint64_t* uncertified_count, void* stream);
+int reid_knn_tau_floor(float* tau, uint32_t* tau_ord, int64_t m, int64_t N, void* stream);
+int reid_knn_candidates_sym_tiles(const void* xh, int64_t N, int64_t D, int scale_log2, const float* tau,
+                                  const int32_t* tiles, int64_t n_tiles, int cap, uint64_t* cand, int32_t* cand_cnt,
+                                  int reset_counts, void* stream);
+int reid_knn_list_tau(const uint64_t* cand, const int32_t* cand_cnt, int cap, int64_t row0, int64_t n_rows, int r,
+                      float* tau, uint32_t* tau_ord, void* stream);
 
 /* fp32 features -> scaled fp16 operand; max_sqnorm_out (optional, TWO floats) = { max_i ||x_i||^2, min_i ||x_i||^2 }:
  * the maximum scales the fp16 rounding bound  |approx - exact| <= 2^-10 ||x_i|| ||x_j||, the pair tells the caller

@@ -51,6 +51,9 @@ SIGNATURES = {
     "reid_knn_sample_tau_emit": (_I, [_P, _P, _P, _I, _L, _I, _P, _P, _P, _P, _I, _L, _P]),
     "reid_features_to_half_gather": (_I, [_P, _P, _L, _L, _I, _P, _P, _P]),
     "reid_knn_candidates_tc_abt": (_I, [_P, _L, _P, _L, _L, _I, _L, _L, _I, _I, _I, _P, _P, _P, _I, _P, _P, _P, _I, _P]),
+    "reid_knn_candidates_sym_tiles": (_I, [_P, _L, _L, _I, _P, _P, _L, _I, _P, _P, _I, _P]),
+    "reid_knn_tau_floor": (_I, [_P, _P, _L, _L, _P]),
+    "reid_knn_list_tau": (_I, [_P, _P, _I, _L, _L, _I, _P, _P, _P]),
     "reid_knn_rescore_mapped": (_I, [_P, _L, _L, _L, _L, _P, _P, _P, _I, _I, _L, _I, _F, _P, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "reid_reciprocal_masks": (_I, [_P, _L, _I, _I, _L, _L, _P, _P]),
     "reid_reciprocal_masks2": (_I, [_P, _L, _I, _I, _I, _L, _L, _P, _P, _P]),

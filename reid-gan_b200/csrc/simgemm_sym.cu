@@ -457,6 +457,76 @@ __global__ void __launch_bounds__(kTauWarps * 32) sample_tau_kernel(const unsign
   }
 }
 
+// Provisional threshold of the non-sample rows in the sample-first layout: tau' = the smallest of the sample rows'
+// thresholds tau_ord[0, m) (a row that scores like the weakest sample row still finds r sample scores above it),
+// written to tau[m, N) and tau_ord[m, N).  Every block finds the minimum and writes its grid-stride share.
+constexpr int kFloorThreads = 1024;
+__global__ void __launch_bounds__(kFloorThreads) tau_floor_kernel(float* __restrict__ tau, uint32_t* __restrict__ tau_ord,
+                                                                  int64_t m, int64_t N) {
+  __shared__ uint32_t s_min;
+  if (threadIdx.x == 0) s_min = 0xffffffffu;
+  uint32_t v = 0xffffffffu;
+  for (int64_t i = threadIdx.x; i < m; i += kFloorThreads) v = min(v, tau_ord[i]);
+  v = __reduce_min_sync(kFull, v);
+  __syncthreads();
+  if (lane_id() == 0) atomicMin(&s_min, v);
+  __syncthreads();
+  const uint32_t T = s_min;
+  const float t = T ? ord_float(T) : -INFINITY;
+  for (int64_t i = m + (int64_t)blockIdx.x * kFloorThreads + threadIdx.x; i < N; i += (int64_t)gridDim.x * kFloorThreads) {
+    tau[i] = t;
+    tau_ord[i] = T;
+  }
+}
+
+// Threshold of a non-sample row in the sample-first layout, after the symmetric kernel has run the sample block column
+// with tau[row] = tau' (tau_floor_kernel): the row's list then holds exactly its sample scores above tau', and
+//   tau[row] = max(tau', r-th best of them)   when at least r are listed,   tau' otherwise.
+// Sound either way: an unlisted sample column scored <= tau' <= tau[row].  One warp per row; as in sample_tau_kernel the
+// search resolves the top 16 bits of the image (rounded down: a few more columns get through).  Only the first
+// min(count, kListTauMax) entries are read: a subset can only lower the r-th best (an overflowed list un-certifies the
+// row in any case).
+constexpr int kListTauMax = 1024;
+__global__ void __launch_bounds__(kTauWarps * 32) list_tau_kernel(const unsigned long long* __restrict__ cand,
+                                                                 const int32_t* __restrict__ cand_cnt, int cap, int64_t row0,
+                                                                 int64_t n_rows, int r, float* __restrict__ tau,
+                                                                 uint32_t* __restrict__ tau_ord) {
+  const int w = threadIdx.x >> 5, lane = lane_id();
+  const int64_t row = row0 + (int64_t)blockIdx.x * kTauWarps + w;
+  if (row >= row0 + n_rows) return;
+  const uint32_t floor_ord = tau_ord[row];
+  const int n = min(min(cand_cnt[row], cap), kListTauMax);
+  if (n < r) return;                                  // tau' stays
+  const unsigned long long* src = cand + row * (int64_t)cap;
+  auto search = [&](auto per_tag) {
+    constexpr int kPer = decltype(per_tag)::value;
+    uint32_t o[kPer];
+#pragma unroll
+    for (int u = 0; u < kPer; ++u) {
+      const int t = u * 32 + lane;
+      o[u] = t < n ? float_ord(__uint_as_float((uint32_t)(src[t] >> 32))) : 0u;
+    }
+    uint32_t T_ = 0;
+#pragma unroll 1
+    for (int bit = 31; bit >= 16; --bit) {
+      const uint32_t c2 = T_ | (1u << bit);
+      int c = 0;
+#pragma unroll
+      for (int u = 0; u < kPer; ++u) c += o[u] >= c2;
+      c = __reduce_add_sync(kFull, c);
+      if (c >= r) T_ = c2;
+    }
+    return T_;
+  };
+  const uint32_t T = n <= 64 ? search(std::integral_constant<int, 2>{})
+                     : n <= 256 ? search(std::integral_constant<int, 8>{})
+                                : search(std::integral_constant<int, kListTauMax / 32>{});
+  if (lane == 0 && T > floor_ord) {
+    tau[row] = ord_float(T);
+    tau_ord[row] = T;
+  }
+}
+
 }  // namespace tc
 }  // namespace reid
 
@@ -562,5 +632,35 @@ int reid_knn_candidates_sym(const void* xh, int64_t N, int64_t D, int scale_log2
 int reid_knn_candidates_sym_wide(const void* xh, int64_t N, int64_t D, int scale_log2, const float* tau, const int32_t* units,
                                  int64_t n_units, int cap, uint64_t* cand, int32_t* cand_cnt, int reset_counts, void* stream) {
   return launch_sym(2, xh, N, D, scale_log2, tau, units, n_units, cap, cand, cand_cnt, reset_counts, stream);
+}
+
+int reid_knn_candidates_sym_tiles(const void* xh, int64_t N, int64_t D, int scale_log2, const float* tau, const int32_t* tiles,
+                                  int64_t n_tiles, int cap, uint64_t* cand, int32_t* cand_cnt, int reset_counts, void* stream) {
+  return launch_sym(1, xh, N, D, scale_log2, tau, tiles, n_tiles, cap, cand, cand_cnt, reset_counts, stream);
+}
+
+int reid_knn_tau_floor(float* tau, uint32_t* tau_ord, int64_t m, int64_t N, void* stream) {
+  using namespace reid;
+  REID_CHECK_ARG(tau && tau_ord, "reid_knn_tau_floor: NULL pointer");
+  REID_CHECK_ARG(m >= 1 && m <= N, "reid_knn_tau_floor: need 1 <= m <= N (m=%lld N=%lld)", (long long)m, (long long)N);
+  if (m == N) return REID_OK;
+  const int64_t blocks = (N - m + 4 * tc::kFloorThreads - 1) / (4 * tc::kFloorThreads);
+  tc::tau_floor_kernel<<<(unsigned)(blocks < 148 ? blocks : 148), tc::kFloorThreads, 0, (cudaStream_t)stream>>>(tau, tau_ord, m,
+                                                                                                             N);
+  REID_LAUNCH_CHECK();
+  return REID_OK;
+}
+
+int reid_knn_list_tau(const uint64_t* cand, const int32_t* cand_cnt, int cap, int64_t row0, int64_t n_rows, int r, float* tau,
+                      uint32_t* tau_ord, void* stream) {
+  using namespace reid;
+  REID_CHECK_ARG(cand && cand_cnt && tau && tau_ord, "reid_knn_list_tau: NULL pointer");
+  REID_CHECK_ARG(cap >= 1 && row0 >= 0 && n_rows >= 0 && r >= 1, "reid_knn_list_tau: bad arguments (cap=%d row0=%lld n_rows=%lld r=%d)",
+                 cap, (long long)row0, (long long)n_rows, r);
+  if (n_rows == 0) return REID_OK;
+  tc::list_tau_kernel<<<(unsigned)((n_rows + tc::kTauWarps - 1) / tc::kTauWarps), tc::kTauWarps * 32, 0, (cudaStream_t)stream>>>(
+      (const unsigned long long*)cand, cand_cnt, cap, row0, n_rows, r, tau, tau_ord);
+  REID_LAUNCH_CHECK();
+  return REID_OK;
 }
 }

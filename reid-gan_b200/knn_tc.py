@@ -232,16 +232,34 @@ def _tile_order_from(n_t, first, dev):
     return _tile_cache[key_]
 
 
+def _sample_block_tiles(n_t, s_t, dev):
+    """The tiles (I, J), I < s_t <= J: the block column of the sample against the other rows, column block by column
+    block (the s_t sample blocks stay in L2, every other block is read by s_t tiles in a row).  Cached."""
+    key_ = ("sample", n_t, s_t, str(dev))
+    if key_ not in _tile_cache:
+        out = [(i, j) for j in range(s_t, n_t) for i in range(s_t)]
+        _tile_cache[key_] = torch.tensor(out, dtype=torch.int32).reshape(-1, 2).to(dev).contiguous()
+    return _tile_cache[key_]
+
+
+def _tau_floor(tau, tau_ord, m, N, sp):
+    """tau[m:] = tau_ord[m:] = tau', the provisional threshold of the rows outside the sample: the smallest sample-row
+    threshold (reid_knn_tau_floor).  A higher choice (the 8th or 32nd smallest of 2,048) measured no faster at
+    N = 32,621: lists 2-3 % shorter, the same re-score time, and up to 30x more rows left at tau'."""
+    call("reid_knn_tau_floor", ptr(tau), ptr(tau_ord), m, N, sp)
+
+
 def _candidates_sym_sf(x, N, D, sp, dev, k, msq):
     """Symmetric search in the sample-first layout.  The fp16 operand is written with the m threshold-sample rows first,
-    so `all rows x sample` IS the block column [0, m) of the similarity matrix:
+    so the rows against the sample are the block column [0, m) of the similarity matrix:
       A. sample rows x sample  -> thresholds of the sample rows; their listed scores above the threshold are their
-         candidates among the sample (reid_knn_sample_tau_emit);
-      B. other rows x sample   -> thresholds of the other rows + their candidates among the sample (same), and, score
-         by score, the transposed direction against the sample rows' thresholds from A (reid_knn_candidates_tc_abt);
+         candidates among the sample (reid_knn_sample_tau_emit).  Then tau' (_tau_floor) for the other rows;
+      B. the symmetric kernel on the tiles (I, J), I < m / 256 <= J (reid_knn_candidates_sym_tiles): sample row i lists
+         column j above its threshold, row j lists sample column i above tau'.  reid_knn_list_tau then raises tau' of
+         row j to the r-th best of its listed sample scores (they are all of them above tau');
       C. the symmetric kernel on the tiles (I, J), m / 256 <= I <= J, appending to the same lists.
     Every pair of rows is scored exactly once; all lists and thresholds are indexed by POSITION (reid_knn_rescore_mapped
-    translates).  Returns (cand, cnt, tau_ord, cap, stats, xh, maps)."""
+    translates).  Needs m % 256 == 0 and N - m >= 256.  Returns (cand, cnt, tau_ord, cap, stats, xh, maps)."""
     m = sample_size(N, k)
     pos_of, orig_of = _sample_first_maps(N, m, dev)
     xh = torch.empty((N, D), dtype=torch.float16, device=dev)
@@ -252,9 +270,6 @@ def _candidates_sym_sf(x, N, D, sp, dev, k, msq):
     tau_ord = torch.empty(N, dtype=torch.int32, device=dev)
     n_rest = N - m
     splits_a = prepass_splits(m, m, max_splits=8)
-    pre = torch.empty(max(n_rest, 1) * 2 * TC_CAP, dtype=torch.int64, device=dev)
-    pre_cnt = torch.zeros(max(n_rest, 1) * 2, dtype=torch.int32, device=dev)
-    pre_tau = torch.empty(max(n_rest, 1), dtype=torch.int32, device=dev)
     # fp16 operand, sample rows first.  Phase A needs only those: it runs on a forked stream (64 tile units for 74 CTA
     # pairs, tensor bound) under the conversion of the other rows (HBM bound); with its own list buffers.
     call("reid_sqnorm_range_reset", ptr(msq), sp)
@@ -272,20 +287,18 @@ def _candidates_sym_sf(x, N, D, sp, dev, k, msq):
              ptr(pre_a_tau), 1, None, None, None, 0, sp_a)
         call("reid_knn_sample_tau_emit", ptr(pre_a), ptr(pre_a_cnt), ptr(pre_a_tau), 2 * splits_a, m, r, ptr(tau), ptr(tau_ord),
              ptr(cand), ptr(cnt), SYM_CAP, 0, sp_a)
-    if n_rest > 0:
-        call("reid_features_to_half_gather", ptr(x), ptr(orig_of[m:]), n_rest, D, SCALE_LOG2, ptr(xh[m:]), ptr(msq), sp)
+        _tau_floor(tau, tau_ord, m, N, sp_a)
+    call("reid_features_to_half_gather", ptr(x), ptr(orig_of[m:]), n_rest, D, SCALE_LOG2, ptr(xh[m:]), ptr(msq), sp)
     main.wait_stream(side)
-    # B: the other rows against the sample, both directions
-    if n_rest > 0:
-        call("reid_knn_candidates_tc_abt", ptr(xh), N, ptr(xh), m, D, SCALE_LOG2, m, N, -r, 1, 2, ptr(pre), ptr(pre_cnt),
-             ptr(pre_tau), 1, ptr(tau), ptr(cand), ptr(cnt), SYM_CAP, sp)
-        call("reid_knn_sample_tau_emit", ptr(pre), ptr(pre_cnt), ptr(pre_tau), 2, n_rest, r, ptr(tau[m:]), ptr(tau_ord[m:]),
-             ptr(cand), ptr(cnt), SYM_CAP, m, sp)
-    # C: the rest of the upper triangle
+    # B: the sample block column, both directions, then the other rows' thresholds
     n_t = (N + 255) // 256
+    b_tiles = _sample_block_tiles(n_t, m // 256, dev)
+    call("reid_knn_candidates_sym_tiles", ptr(xh), N, D, SCALE_LOG2, ptr(tau), ptr(b_tiles), b_tiles.shape[0], SYM_CAP, ptr(cand),
+         ptr(cnt), 0, sp)
+    call("reid_knn_list_tau", ptr(cand), ptr(cnt), SYM_CAP, m, n_rest, r, ptr(tau), ptr(tau_ord), sp)
+    # C: the rest of the upper triangle
     tiles = _tile_order_from(n_t, m // 256, dev)
-    if tiles.shape[0]:
-        candidates_sym_launch(xh, N, D, tau, tiles, SYM_CAP, cand, cnt, 0, sp)
+    candidates_sym_launch(xh, N, D, tau, tiles, SYM_CAP, cand, cnt, 0, sp)
     return cand, cnt, tau_ord, SYM_CAP, dict(sample=m, tiles=int(tiles.shape[0]), layout="sample-first"), xh, (pos_of, orig_of)
 
 
